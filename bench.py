@@ -145,7 +145,8 @@ def make_idct_workload(torch, L, stream, rank):
 
     return {
         "name": "batched simple_idct_put 8x8, 2^20 dense int16 blocks per GPU -> 8192x8192 u8 frame",
-        "run": run, "run_e2e": run_e2e, "verify": verify, "pixels": N_BLOCKS * 64, "alg_bytes": N_BLOCKS * IDCT_BYTES_PER_BLOCK,
+        "run": run, "run_e2e": run_e2e, "verify": verify, "outputs": lambda i: {"frame": d_frame[i % nbuf]},
+        "pixels": N_BLOCKS * 64, "alg_bytes": N_BLOCKS * IDCT_BYTES_PER_BLOCK,
         "launches_per_step": 1, "kernel": "simple_idct_kernel<0,false>",  "dtype": "int32 (int16 in, u8 out)",
         "h2d": N_BLOCKS * 128, "d2h": rows * stride,
         "l2": "3 rotating 192 MiB buffer sets (inputs larger than the 126 MB L2)",
@@ -224,7 +225,8 @@ def make_sws_workload(torch, L, stream, rank):
 
     return {
         "name": "sws_scale 3840x2160 yuv420p->rgb24 bicubic|accurate_rnd|bitexact, %d frames per launch per GPU" % K,
-        "run": run, "run_e2e": run_e2e, "verify": verify, "pixels": w * h * K, "alg_bytes": int(w * h * K * SWS_BYTES_PER_PIXEL),
+        "run": run, "run_e2e": run_e2e, "verify": verify, "outputs": lambda i: {"rgb24": d_o[i % nbuf].view(K, h, w * 3)},
+        "pixels": w * h * K, "alg_bytes": int(w * h * K * SWS_BYTES_PER_PIXEL),
         "launches_per_step": 1, "kernel": "sws_fused_rgb24_tma_kernel", "dtype": "int32 (u8 in, u8 out)",
         "h2d": int(w * h * 1.5) * K, "d2h": osz * K,
         "l2": "2 rotating %d MiB buffer sets (inputs+outputs larger than the 126 MB L2)" % ((ysz + 2 * csz + osz) * K >> 20),
@@ -255,7 +257,8 @@ def make_sws_up_workload(torch, L, stream, rank):
 
     return {
         "name": "sws_scale 1920x1080 -> 3840x2160 yuv420p->rgb24 bicubic|accurate_rnd|bitexact (true rescale), %d frames per step" % K,
-        "run": run, "run_e2e": None, "pixels": dw * dh * K, "alg_bytes": int((sw * sh * 1.5 + dw * dh * 3) * K),
+        "run": run, "run_e2e": None, "outputs": lambda i: {"rgb24": d_o.view(K, dh, dw * 3)},
+        "pixels": dw * dh * K, "alg_bytes": int((sw * sh * 1.5 + dw * dh * 3) * K),
         "launches_per_step": 1, "kernel": "sws_tile_rgb24_kernel", "dtype": "int32 (u8 in, u8 out)", "h2d": 0, "d2h": 0,
         "l2": "%d MiB of output per step" % (osz * K >> 20), "keep": (d_y, d_u, d_v, d_o, ctx),
     }
@@ -351,6 +354,7 @@ def make_h264_workload(torch, L, stream, rank):
     return {
         "name": NAMES["h264"],
         "run": run, "run_e2e": None, "verify": verify, "pixels": W * H * P, "alg_bytes": int(n_mb * 2.37e3),
+        "outputs": lambda i: {"y": d_y.view(P, H, W), "cb": d_cb.view(P, H // 2, W // 2), "cr": d_cr.view(P, H // 2, W // 2)},
         "launches_per_step": 4 * G, "kernel": "h264_mc_kernel_v2", "dtype": "int32 (u8 / int16 in, u8 out)", "h2d": 0, "d2h": 0,
         "l2": "%d pictures (%d MC partitions each) per step: %d MB of pixels + %d MB of coefficients, larger than the 126 MB L2" % (P, mc1.shape[0], P * W * H * 3 // 2 >> 20, d_coef0.numel() >> 20),
         "keep": (d_refs, d_planes_g, d_mc, d_res, d_nnz, d_dbk, d_coef0, d_coef, d_y, d_cb, d_cr, d_prog, side, refilled, consumed, chains, fork, joined),
@@ -381,7 +385,7 @@ def make_h264_decide_workload(torch, L, stream, rank):
     per_mb = 4 + 1 + 48 + 2 + 2 + 2 * 64 + 2 * 4 + 104
     return {
         "name": "H.264 deblocking decisions (bS, alpha, beta, tc0) for %d stacked 1080p B pictures of 8 slices" % P,
-        "run": run, "run_e2e": None, "pixels": 256 * n, "alg_bytes": n * per_mb,
+        "run": run, "run_e2e": None, "outputs": lambda i: {"deblock_records": d_out.view(n, 104)}, "pixels": 256 * n, "alg_bytes": n * per_mb,
         "launches_per_step": 1, "kernel": "h264_deblock_params_kernel", "dtype": "int32 (decoder side information in, records out)",
         "h2d": 0, "d2h": 0, "l2": "%d MB of side information + records per step" % (n * per_mb >> 20), "keep": (keep, d_out, info),
     }
@@ -416,7 +420,8 @@ def make_dequant_idct_workload(torch, L, stream, rank):
 
     return {
         "name": "fused dct_unquantize_mpeg2_intra (bitexact) + simple_idct_put, 2^20 blocks per GPU -> 8192x8192 u8 frame",
-        "run": run, "run_e2e": None, "pixels": N_BLOCKS * 64, "alg_bytes": N_BLOCKS * (IDCT_BYTES_PER_BLOCK + 4),
+        "run": run, "run_e2e": None, "outputs": lambda i: {"frame": d_frame[i % nbuf]},
+        "pixels": N_BLOCKS * 64, "alg_bytes": N_BLOCKS * (IDCT_BYTES_PER_BLOCK + 4),
         "launches_per_step": 1, "kernel": "simple_idct_kernel<0,false,4,false,4>", "dtype": "int32 (int16 levels in, u8 out)",
         "h2d": 0, "d2h": 0, "l2": "3 rotating 196 MiB buffer sets", "keep": (d_blocks, d_rec, d_frame, t),
     }
@@ -444,7 +449,8 @@ def make_idct10_workload(torch, L, stream, rank):
 
     return {
         "name": "batched simple_idct_put_10 (10-bit), 2^20 int16 blocks per GPU -> 8192x8192 16-bit frame",
-        "run": run, "run_e2e": None, "pixels": N_BLOCKS * 64, "alg_bytes": N_BLOCKS * 384,
+        "run": run, "run_e2e": None, "outputs": lambda i: {"frame": d_frame[i % nbuf], "blocks": d_blocks[i % nbuf]},
+        "pixels": N_BLOCKS * 64, "alg_bytes": N_BLOCKS * 384,
         "launches_per_step": 1, "kernel": "simple_idct10_staged_kernel<0>", "dtype": "int32 (int16 in, u16 out)", "h2d": 0, "d2h": 0,
         "l2": "2 rotating 384 MiB buffer sets (the row pass is written back over the coefficients, as the C functions leave it)",
         "keep": (d_blocks0, d_blocks, d_off, d_frame),
@@ -491,6 +497,8 @@ def make_h264_hbd_workload(torch, L, stream, rank):
     return {
         "name": "H.264 1080p DSP path on 10-bit pictures (functional kernels): MC + residual + deblock, %d stacked 64-slice pictures per step" % P,
         "run": run, "run_e2e": None, "pixels": P * W * H, "alg_bytes": n * (2 * 768 + 3 * 1536 + 104 + 1536),
+        "outputs": lambda i: {"y": d_y.view(torch.int16).view(P, H, W), "cb": d_cb.view(torch.int16).view(P, H // 2, W // 2),
+                              "cr": d_cr.view(torch.int16).view(P, H // 2, W // 2)},
         "launches_per_step": 4, "kernel": "h264_deblock_generic_kernel", "dtype": "int32 (u16 samples, int32 coefficients)", "h2d": 0, "d2h": 0,
         "l2": "%d MiB of pictures + coefficients per step" % ((P * W * H * 3 + n * 3072) >> 20),
         "keep": (d_refs, d_planes, d_mc, d_res, d_nnz, d_dbk, d_coef0, d_coef, d_y, d_cb, d_cr),
@@ -534,6 +542,7 @@ def make_h264_intra_workload(torch, L, stream, rank):
     return {
         "name": "H.264 intra reconstruction wavefront: %d all-intra 1080p pictures per step (4x4 / 8x8 / 16x16 mix)" % P,
         "run": run, "run_e2e": None, "pixels": W * H * P, "alg_bytes": n_mb * (768 * 2 + 384 + 120 + 24),
+        "outputs": lambda i: {"y": d_y.view(P, H, W), "cb": d_cb.view(P, H // 2, W // 2), "cr": d_cr.view(P, H // 2, W // 2)},
         "launches_per_step": 1, "kernel": "h264_intra_kernel", "dtype": "int32 (u8 / int16 in, u8 out)", "h2d": 0, "d2h": 0,
         "l2": "%d MB of coefficients + pixels per step" % (n_mb * (768 * 2 + 384) >> 20),
         "keep": (d_rec, d_nnz, d_coef0, d_coef, d_y, d_cb, d_cr, d_prog, side, refilled, consumed),
@@ -547,15 +556,25 @@ def make_fft_workload(torch, L, stream, rank):
     nb, T = 10, 32768
     g = torch.Generator(device="cuda"); g.manual_seed(1 + rank)
     bufs = [torch.randn(T * (1 << nb) * 2, generator=g, device="cuda", dtype=torch.float32) for _ in range(2)]
+    inputs = [b.clone() for b in bufs]
 
     def run(i):
         L.check(lib.ff_fft_batch_cuda(nb, 0, bufs[i & 1].data_ptr(), T, stream), "fft")
 
+    def outputs(i):
+        """the step's transform applied to its buffer's original contents: the timed buffers are transformed over and over
+        without normalisation and soon hold inf / NaN"""
+        out = inputs[i & 1].clone()
+        L.check(lib.ff_fft_batch_cuda(nb, 0, out.data_ptr(), T, stream), "fft")
+        torch.cuda.synchronize()
+        return {"transforms": out.view(T, 1 << nb, 2)}
+
     return {
         "name": "FFTContext fft_permute + fft_calc: %d x %d-point complex float transforms per step" % (T, 1 << nb),
-        "run": run, "run_e2e": None, "pixels": T * (1 << nb), "alg_bytes": T * (1 << nb) * 16,
+        "run": run, "run_e2e": None, "outputs": outputs,
+        "pixels": T * (1 << nb), "alg_bytes": T * (1 << nb) * 16,
         "launches_per_step": 1, "kernel": "fft_kernel", "dtype": "f32 (complex)", "h2d": 0, "d2h": 0,
-        "l2": "2 rotating 256 MiB buffers; the metric counts complex points as pixels", "keep": (bufs,),
+        "l2": "2 rotating 256 MiB buffers; the metric counts complex points as pixels", "keep": (bufs, inputs),
     }
 
 
@@ -583,7 +602,8 @@ def make_me_workload(torch, L, stream, rank):
 
     return {
         "name": "me_cmp pix_abs16 SAD full search, 1920x1088, range 16, whole frame per GPU",
-        "run": run, "run_e2e": None, "verify": verify, "pixels": w * h, "alg_bytes": 2 * w * h + 12 * n_mb,
+        "run": run, "run_e2e": None, "verify": verify, "outputs": lambda i: {"motion": d_out.view(n_mb, 3)},
+        "pixels": w * h, "alg_bytes": 2 * w * h + 12 * n_mb,
         "launches_per_step": 1, "kernel": "full_search_kernel", "dtype": "u8 (vabsdiff4)", "h2d": 0, "d2h": 0,
         "l2": "4 MB working set, ALU/shared-memory bound (2.27 G abs-diff-accumulate per frame), HBM fraction reported for completeness",
         "keep": (d_cur, d_ref, d_out),
@@ -629,6 +649,7 @@ def make_me_sharded_workload(torch, dist, L, stream, rank, world):
     return {
         "name": "me_cmp pix_abs16 SAD full search, 1920x1088, range 16, frame-shard over %d GPUs + ncclAllGather of the motion field" % world,
         "run": run, "run_e2e": None, "verify": verify, "scaling": "strong", "pixels": w * h, "alg_bytes": 2 * w * h + 12 * mb_w * mb_h,
+        "outputs": lambda i: {"motion": d_all.view(world, rows_max * mb_w, 3)},
         "launches_per_step": 1, "kernel": "full_search_kernel", "dtype": "u8 (vabsdiff4)", "h2d": 0, "d2h": 0,
         "l2": "4 MB working set, ALU/shared-memory bound (2.27 G abs-diff-accumulate per frame), HBM fraction reported for completeness",
         "keep": (d_cur, d_ref, d_loc, d_all),
@@ -678,6 +699,27 @@ def time_e2e(torch, dist, wl, steps, warmup, world):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         sec = float(t.item())
     return sec
+
+
+DUMP_BYTES = 60 << 20         # under 64 MB with the .npy headers
+DUMP_SEED = 20261017
+
+
+def dump_outputs(torch, outputs, directory):
+    """Writes each array of `outputs` (device tensors) to <directory>/<name>.npy: float32, or float64 where the data is.  An array
+    larger than its share of DUMP_BYTES is written as a sample at positions drawn from DUMP_SEED: the same positions for the same
+    arguments, so two builds can be compared value for value."""
+    os.makedirs(directory, exist_ok=True)
+    for name, t in outputs.items():
+        flat = t.reshape(-1)
+        ftype = torch.float64 if t.dtype == torch.float64 else torch.float32
+        share = DUMP_BYTES // len(outputs) // (8 if ftype == torch.float64 else 4)
+        if flat.numel() > share:
+            pos = np.sort(np.random.default_rng(DUMP_SEED).integers(0, flat.numel(), share))
+            flat = flat[torch.from_numpy(pos).to(flat.device)]
+        else:
+            flat = flat.reshape(t.shape)
+        np.save(os.path.join(directory, name + ".npy"), flat.to(ftype).cpu().numpy())
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -855,6 +897,7 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary workloads and the CPU baselines")
     ap.add_argument("--no-verify", action="store_true", help="skip the post-timing comparison with the CPU checker")
     ap.add_argument("--tune", action="append", default=[], help="kernel-variant knob key=value (avb200_set_tuning), profiling only")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last step to DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -924,6 +967,8 @@ def main():
         st = steps if idx == 0 else max(5, min(steps, 30))   # the secondaries get a shorter timed region
         sampler = ClockSampler(local_rank) if rank == 0 else None
         ms = time_gpu(torch, dist, wl, st, warmup, world, sampler)
+        if args.dump_outputs and idx == 0 and rank == 0:
+            dump_outputs(torch, wl["outputs"](warmup + st - 1), args.dump_outputs)
         e2e_steps = max(1, min(st, 5))
         e2e_sec = time_e2e(torch, dist, wl, e2e_steps, warmup, world) if wl["run_e2e"] else None
         verified = None

@@ -2,6 +2,7 @@
 ctypes binding lists the same set, the header compiles as plain C, and the table structs are layout-identical
 to the reference's (sizes/offsets from oracle/_ref when it is built).  No compute entry point is called."""
 import ctypes as C
+import json
 import os
 import re
 import subprocess
@@ -46,13 +47,13 @@ def test_header_is_plain_c_and_layout_matches_reference(built, tmp_path):
     assert C.sizeof(tables.QpelDSPContext) == mine[30] and tables.QpelDSPContext.put_no_rnd_qpel_pixels_tab.offset == mine[31]
     from oracle import loader
     r = loader.ref()
-    if r is None:
-        pytest.skip("oracle/_ref not built here")
-    out = np.zeros(64, np.int32)
-    r.lib.ref_abi_info.restype = C.c_int
-    n = r.lib.ref_abi_info(out.ctypes.data_as(C.c_void_p), 64)
-    assert n == len(mine)
-    assert list(out[:n]) == mine
+    if r is None:       # the reference's sizes and offsets (ref_abi_info), recorded where oracle/_ref was built
+        ref_abi = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_abi.json")))
+    else:
+        out = np.zeros(64, np.int32)
+        r.lib.ref_abi_info.restype = C.c_int
+        ref_abi = out[:r.lib.ref_abi_info(out.ctypes.data_as(C.c_void_p), 64)].tolist()
+    assert ref_abi == mine
 
 
 def test_no_gpu_means_loud_failure(built):

@@ -6,14 +6,11 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from oracle import loader
 import enc_cases
 
-pytestmark = pytest.mark.skipif(loader.ref() is None, reason="oracle/_ref not built")
 
-
-def test_quantiser_matrices_match_ff_convert_matrix():
-    port, ref = loader.port(), loader.ref()
+def test_quantiser_matrices_match_ff_convert_matrix(orc, refo):
+    port, ref = orc, refo
     T = enc_cases.Tables(1)
     for label, st in enc_cases.states(T):
         got = [np.zeros(64, np.int32), np.zeros(64, np.int32), np.zeros(64, np.uint8)]
@@ -25,8 +22,8 @@ def test_quantiser_matrices_match_ff_convert_matrix():
 
 
 @pytest.mark.parametrize("kind", sorted(enc_cases.KINDS))
-def test_port_matches_reference(kind):
-    port, ref = loader.port(), loader.ref()
+def test_port_matches_reference(orc, refo, kind):
+    port, ref = orc, refo
     T = enc_cases.Tables(2)
     n = 24
     cur, rf = enc_cases.block_pairs(n, seed=kind)
